@@ -13,6 +13,7 @@ timed region, 16 B result read back per step); `e2e_evaluate` is eval_lm.evaluat
 reference-layout data directory in tmpfs (mmap slicing, collater, staging, scoring).  Prints ONE JSON line on rank 0.
 
   python bench.py --gpus N --scaling strong   # a fixed corpus sharded over the ranks through evaluate() (extra evidence)
+  python bench.py ... --dump-outputs DIR      # also write the last timed step's outputs as DIR/*.npy (compare two builds)
 """
 import argparse
 import json
@@ -59,7 +60,33 @@ def parse():
     p.add_argument("--ncu-range", action="store_true",
                    help="after warm-up run ONE resident step inside cudaProfilerStart/Stop and exit "
                         "(use with `ncu --profile-from-start off`); prints no bench line")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps write what the last one returned as DIR/<name>.npy (rank 0): logprob [B, L] and "
+                        "gcn_feat [B, L, d] in float32, nll_acc (sum log p, tokens over every step so far) in float64.  The "
+                        "inputs are seeded, so two builds run with the same arguments can be compared output for output")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    return a
+
+
+DUMP_LIMIT = (64 << 20) - (64 << 10)          # 64 MB in all, with room for the .npy headers
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> tensor, written smallest first as <out_dir>/<name>.npy.  An array that would take the total past
+    DUMP_LIMIT is written as a fixed, seeded sample (in order) of its rows over the last dimension, [n_sampled, last_dim]."""
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_LIMIT
+    for name, t in sorted(arrays.items(), key=lambda kv: kv[1].numel()):
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.nbytes > left:
+            a = a.reshape(-1, a.shape[-1])
+            keep = np.random.RandomState(0).choice(a.shape[0], left // (a.itemsize * a.shape[1]), replace=False)
+            a = a[np.sort(keep)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        left -= a.nbytes
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -357,7 +384,11 @@ def main():
         return float(ms.item())
 
     eager = lambda i: runner.step_resident(dev_batches[i % NB])
-    resident = lambda i: runner.step_resident(dev_batches[i % NB], cuda_graph=args.cuda_graph)
+    last = {}
+
+    def resident(i):
+        last["out"] = runner.step_resident(dev_batches[i % NB], cuda_graph=args.cuda_graph)
+
     host = lambda i: runner.step_host(host_batches[i % NB], cuda_graph=args.cuda_graph)
 
     eager(0)                                                         # one-time weight preparation (folds, fp16 splits) happens here
@@ -378,6 +409,9 @@ def main():
     ms = timed(resident, args.steps)
     launches = launches_per_step * args.steps
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:         # before the host leg: it replays the same CUDA graph into the same buffers
+        lp, _, _, (feat, _) = last["out"]
+        dump_outputs(args.dump_outputs, {"logprob": lp, "gcn_feat": feat, "nll_acc": runner.acc})
     for i in range(2):
         host(i)
     # e2e: K steps through the runner's host-input loop -- per step: H2D of that step's pinned inputs (double-buffered on a
