@@ -104,6 +104,10 @@ SIGNATURES = {
     "gnnlm_axpy_f32": (_i32, [_p, _i64, _p, _i64, _i64, _p, _i64, _f32, _p]),
     "gnnlm_scatter_add_rows": (_i32, [_p, _i64, _p, _i64, _p, _i64, _p, _i64, _p]),
     "gnnlm_knn_sims_pq": (_i32, [_p, _i64, _i32, _p, _i64, _p, _i64, _i32, _i32, _p, _p, _p, _i64, _i32, _p, _i32, _p, _i64, _p]),
+    "gnnlm_knn_filter_f16x3": (_i32, [_p, _i64, _i64, _i64, _p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i64, _p]),
+    "gnnlm_topk_merge": (_i32, [_p, _p, _i64, _i32, _p, _p, _p, _i64, _p, _p]),
+    "gnnlm_knn_key_bias": (_i32, [_p, _i32, _i64, _i64, _i64, _p, _p]),
+    "gnnlm_knn_key_bias_pq": (_i32, [_p, _i64, _i32, _p, _p, _p]),
 }
 
 _lib = None

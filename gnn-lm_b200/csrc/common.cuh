@@ -42,6 +42,18 @@ void set_error(const char* fmt, ...);
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// cudaFuncSetAttribute acts on the current device only, so a one-time set-up is remembered per device (index into a
+// [MAX_DEVICES] flag array) -- a process that drives several GPUs configures each of them.
+constexpr int MAX_DEVICES = 64;
+static inline int device_slot() {
+  int d = 0;
+  if (cudaGetDevice(&d) != cudaSuccess) {
+    cudaGetLastError();
+    d = 0;
+  }
+  return d < MAX_DEVICES ? d : MAX_DEVICES - 1;
+}
+
 __device__ __forceinline__ int64_t live_rows(int64_t cap, const int32_t* dev) {
   if (dev == nullptr) return cap;
   int64_t n = (int64_t)__ldg(dev);

@@ -184,6 +184,56 @@ struct EpiLse {
   int64_t n_tiles;
 };
 
+// Top-k filter of the exact kNN search (gnnlm_knn_filter_f16x3): rows are datastore keys, columns queries.  Nothing is
+// stored per (key, query); only scores s = acc + row_bias[m] above the query's threshold become candidates.
+struct EpiTopk {
+  const float* row_bias;   // [M] (-1/2 ||x||^2 for l2), nullable
+  const float* thr;        // [N] per-query threshold (strict: s > thr)
+  float* cand_s;           // [N, cap]
+  int32_t* cand_id;        // [N, cap]
+  int32_t* cand_cnt;       // [N]: counts every candidate, also past cap (overflow = cand_cnt > cap)
+  int64_t cap;
+  int64_t id_base;         // id of row 0
+};
+
+// One key row per thread.  The 32 thresholds of a chunk sit in one register per lane and are broadcast by shuffle; per
+// column the warp ballots `s > thr`, one lane reserves the slots with a single atomicAdd, and every passing lane writes
+// (s, id) at its rank.  Writes stop at cap; the count keeps growing so that the host sees the overflow.
+__device__ __forceinline__ void epilogue_topk(uint32_t taddr, int64_t m, int64_t M, int64_t n_base, int64_t N, const EpiTopk& et,
+                                              float acc_scale) {
+  const int lane = threadIdx.x & 31;
+  const bool row_ok = m < M;
+  const float rb = (row_ok && et.row_bias) ? __ldg(et.row_bias + m) : 0.f;
+  const int32_t id = (int32_t)(et.id_base + m);
+  const uint32_t below = (1u << lane) - 1u;
+  float v[32];
+#pragma unroll 1
+  for (int c = 0; c < BLOCK_N; c += 32) {
+    const int64_t n0 = n_base + c;
+    if (n0 >= N) break;                                          // warp-uniform
+    const float t_l = n0 + lane < N ? __ldg(et.thr + n0 + lane) : INFINITY;
+    tmem_ld32(taddr + (uint32_t)c, v);
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      const float t = __shfl_sync(0xffffffffu, t_l, j);
+      float s = fmaf(v[j], acc_scale, rb);
+      s = s == 0.f ? 0.f : s;                                    // -0 -> +0: equal scores compare equal in the merge's ordering
+      const bool p = row_ok && s > t;
+      const uint32_t b = __ballot_sync(0xffffffffu, p);
+      if (b) {
+        int base = 0;
+        if (lane == 0) base = atomicAdd(et.cand_cnt + n0 + j, __popc(b));
+        base = __shfl_sync(0xffffffffu, base, 0);
+        const int64_t r = base + __popc(b & below);
+        if (p && r < et.cap) {
+          et.cand_s[(n0 + j) * et.cap + r] = s;
+          et.cand_id[(n0 + j) * et.cap + r] = id;
+        }
+      }
+    }
+  }
+}
+
 // One output row per thread: drain 32-column chunks of this warp's TMEM lane quarter and either store them
 // (bias / residual fused) or fold them into the running (max, sum-exp, picked logit) of the row.
 constexpr int EPI_LD = 36;                                  // padded row of the per-warp 32x32 staging tile (floats)

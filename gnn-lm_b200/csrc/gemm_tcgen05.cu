@@ -621,18 +621,20 @@ __host__ __device__ inline int64_t f16s_causal_tiles(int64_t n_p, int64_t n_n) {
 // The log-sum-exp epilogue (one FFMA + one MUFU.EX2 per logit, online max) paces the K = 64 tail-cluster GEMMs (ncu: a single
 // epilogue warp per scheduler, 31 % issue-slot use, every other warp parked at the final barrier), so the LSE instantiation runs
 // EIGHT epilogue warps -- two per TMEM lane quarter, each reducing half of the tile's columns -- and 384 threads.
-template <bool LSE>
+// TOPK: the kNN filter epilogue (epilogue_topk) instead of a store; its MMAs are always N = 256 wide, so that a score does not
+// depend on how many queries share the launch.
+template <bool LSE, bool TOPK = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSE ? 384 : 256, 1)
     gemm_f16s_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
                      const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_blo, int64_t M_cap,
                      const int32_t* __restrict__ m_dev, int64_t N, int64_t K, EpiStore es, EpiLse el, float acc_scale, int nb,
-                     int64_t c_bs, int64_t r_bs, int causal) {
+                     int64_t c_bs, int64_t r_bs, int causal, EpiTopk et) {
   constexpr int STAGES = F16S_STAGES;
   constexpr uint32_t TX = 2u * F16S_STAGE;                                // both CTAs' four operand tiles -> leader
   // N of the instruction: outputs of at most 128 columns (the P V' GEMM of the causal attention, N = d_k = 128; the narrow tail
   // projections) run N = 128 MMAs -- half the tensor work of a padded 256-column tile.  Each CTA of the pair then supplies
   // N / 2 = 64 rows of W: its TMA box starts at row crank * 64 and only the first 64 rows of its tile are read.
-  const int n_mma = N <= BLOCK_N / 2 ? BLOCK_N / 2 : BLOCK_N;
+  const int n_mma = (!TOPK && N <= BLOCK_N / 2) ? BLOCK_N / 2 : BLOCK_N;
   const uint32_t IDESC = (1u << 4) | ((uint32_t)(n_mma >> 3) << 17) | ((uint32_t)((2 * BLOCK_M) >> 4) << 24);
 
   extern __shared__ uint8_t smem_raw[];
@@ -786,7 +788,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSE ? 384 : 256, 1)
         eb.C = reinterpret_cast<float*>(es.C) + bi * c_bs;
         if (es.residual) eb.residual = reinterpret_cast<const float*>(es.residual) + bi * r_bs;
       }
-      if constexpr (LSE)
+      if constexpr (TOPK)
+        epilogue_topk(taddr, m, M, n_base, N, et, acc_scale);
+      else if constexpr (LSE)
         epilogue_tile<LSE>(taddr, m, M, n_base + half * COLS, n_blk, N, eb, el, epi_smem, acc_scale, COLS,
                            &lse_pair[it & 1][q][lane], half ? 1 : 2, 1 + q);
       else
@@ -913,15 +917,17 @@ static int32_t launch_f16x3(const CUtensorMap& ma, const CUtensorMap& mb, const 
   return 0;
 }
 
-template <bool LSE>
+template <bool LSE, bool TOPK = false>
 static int32_t launch_f16s(const CUtensorMap& mah, const CUtensorMap& mal, const CUtensorMap& mb, const CUtensorMap& mblo,
                            int64_t M, const int32_t* m_dev, int64_t N, int64_t K, const EpiStore& es, const EpiLse& el,
-                           float acc_scale, cudaStream_t st, int nb = 1, int64_t c_bs = 0, int64_t r_bs = 0, int causal = 0) {
+                           float acc_scale, cudaStream_t st, int nb = 1, int64_t c_bs = 0, int64_t r_bs = 0, int causal = 0,
+                           const EpiTopk& et = EpiTopk{}) {
   const size_t smem = (size_t)F16S_STAGES * F16S_STAGE + EPI_SMEM + 1024;
-  static bool attr_set = false;
-  if (!attr_set) {
-    GNNLM_CUDA(cudaFuncSetAttribute(gemm_f16s_kernel<LSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
+  static bool attr_set[MAX_DEVICES] = {};
+  bool& done = attr_set[device_slot()];
+  if (!done) {
+    GNNLM_CUDA(cudaFuncSetAttribute(gemm_f16s_kernel<LSE, TOPK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    done = true;
   }
   static int n_sm = 0;
   if (!n_sm) {
@@ -933,9 +939,9 @@ static int32_t launch_f16s(const CUtensorMap& mah, const CUtensorMap& mal, const
   const int64_t pairs = (causal == 1 ? f16s_causal_tiles(n_p, n_n) : n_p * n_n) * nb;
   const int64_t max_pairs = n_sm / 2;
   const unsigned grid = 2u * (unsigned)(pairs < max_pairs ? pairs : max_pairs);
-  gemm_f16s_kernel<LSE><<<grid, LSE ? 384 : 256, smem, st>>>(mah, mal, mb, mblo, M, m_dev, N, K, es, el, acc_scale, nb, c_bs, r_bs,
-                                                             causal);
-  GNNLM_LAUNCH_CHECK("gemm_f16s");
+  gemm_f16s_kernel<LSE, TOPK><<<grid, LSE ? 384 : 256, smem, st>>>(mah, mal, mb, mblo, M, m_dev, N, K, es, el, acc_scale, nb, c_bs,
+                                                                   r_bs, causal, et);
+  GNNLM_LAUNCH_CHECK(TOPK ? "gemm_f16s_topk" : "gemm_f16s");
   return 0;
 }
 
@@ -1029,6 +1035,21 @@ int32_t gemm_tc_store(const void* A, int32_t a_dtype, int64_t lda, const void* W
   if (math == GNNLM_MATH_TF32X3) return tc::launch<tc::X3, false>(ma, mb, mblo, M, m_dev, N, K, es, el, st);
   if (math == GNNLM_MATH_TF32) return tc::launch<tc::TF32, false>(ma, mb, mblo, M, m_dev, N, K, es, el, st);
   return tc::launch<tc::BF16, false>(ma, mb, mblo, M, m_dev, N, K, es, el, st);
+}
+
+// Top-k filter pass of the exact kNN search: scores of the keys A (split fp16 [M, 2K], rows = ids id_base ..) against the queries
+// (W_hi / W_lo [N, K], scale 1), candidates above thr per query (see EpiTopk).
+int32_t gemm_tc_topk(const void* A, int64_t lda, int64_t M, int64_t id_base, const void* W_hi, const void* W_lo, int64_t ldw,
+                     int64_t N, int64_t K, const float* row_bias, const float* thr, float* cand_s, int32_t* cand_id,
+                     int32_t* cand_cnt, int64_t cap, cudaStream_t st) {
+  if (M == 0) return 0;
+  tc::EpiStore es{};
+  tc::EpiLse el{};
+  const tc::EpiTopk et{row_bias, thr, cand_s, cand_id, cand_cnt, cap, id_base};
+  CUtensorMap mah, mal, mb, mblo;
+  int32_t rc = f16s_maps("gnnlm_knn_filter_f16x3", A, lda, W_hi, W_lo, ldw, M, N, K, &mah, &mal, &mb, &mblo);
+  if (rc) return rc;
+  return tc::launch_f16s<false, true>(mah, mal, mb, mblo, M, nullptr, N, K, es, el, 1.f, st, 1, 0, 0, 0, et);
 }
 
 int32_t gemm_tc_lse(const void* A, int32_t a_dtype, int64_t lda, const void* W, const void* W_lo, float w_scale, int64_t ldw,

@@ -395,11 +395,12 @@ extern "C" int32_t gnnlm_pq_gather_decode_presplit_q8(const uint8_t* codes, int6
                   GNNLM_E_SHAPE, "gnnlm_pq_gather_decode_presplit: out / codebooks must be 16 B aligned, ld_out >= 2*M*8");
   if (n_cap == 0) return 0;
   const size_t smem = (size_t)2 * PQS_MC * 256 * 16;
-  static bool attr_set = false;
-  if (!attr_set) {
+  static bool attr_set[MAX_DEVICES] = {};
+  bool& done = attr_set[device_slot()];
+  if (!done) {
     GNNLM_CUDA(cudaFuncSetAttribute(pq_decode_presplit_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     GNNLM_CUDA(cudaFuncSetAttribute(pq_decode_presplit_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
+    done = true;
   }
   int nodes_per_cta = PQ_NODES_PER_CTA;
   while (nodes_per_cta > 64 && ceil_div(n_cap, nodes_per_cta) * ceil_div(M, PQS_MC) < 296) nodes_per_cta >>= 1;

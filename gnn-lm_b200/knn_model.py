@@ -1,9 +1,10 @@
 """kNN-LM probability -- host-side mirror of knn/knn_model.py:25-217 (KNNModel) for the
-precomputed-neighbour pipeline: the faiss search (get_knns, :87-101) is out of scope, so the
-retrieved (dists, ids) are inputs, exactly as find_knn.py precomputes ids for the graph
+precomputed-neighbour pipeline: the retrieved (dists, ids) are inputs, exactly as find_knn.py precomputes ids for the graph
 (SURVEY.md Q8: the eval script's queries are the same precomputed features find_knn.py searched
-with, hence precomputable).  Everything after the search -- similarity sign, -1 masking, softmax
-over sims/T, the vote on the target or the full-vocabulary scatter -- runs in logprob_knn.cu."""
+with, hence precomputable).  Given a `searcher` (knn_search.KNNSearcher), get_knns searches itself when no results
+were provided, as the reference's get_knns does (exact search instead of the faiss index).  Everything after the search --
+similarity sign, -1 masking, softmax over sims/T, the vote on the target or the full-vocabulary scatter -- runs in
+logprob_knn.cu."""
 from typing import Optional
 
 import torch
@@ -15,13 +16,14 @@ class KNNModel(object):
     def __init__(self, vals: torch.Tensor, vocab_size: Optional[int] = None, metric_type: str = "do_not_recomp_ip",
                  k: int = 1024, dists: Optional[torch.Tensor] = None, knns: Optional[torch.Tensor] = None,
                  keys: Optional[torch.Tensor] = None, pq_codes: Optional[torch.Tensor] = None, quantizer=None,
-                 index_file: str = ""):
+                 index_file: str = "", searcher=None):
         """vals: [N_d] (or [N_d,1]) int16/int32 datastore values resident in HBM (vals.npy);
         dists/knns: optional whole-split precomputed search results [N_split, k] indexed by stream position.
         metric_type `l2` / `ip` recompute the similarities (knn_model.py:159-177) from `keys` ([N_d, d] fp16/fp32 in
         HBM, the reference's keys.npy) or, when the keys only exist PQ-compressed, from `pq_codes` [N_d, M] uint8 +
         `quantizer` (TorchPQCodec) -- then against the decoded keys.  `index_file`: as in the reference, a name
-        containing "cosine" switches on the query / key normalisation (:171-172,181-184), for raw and PQ-decoded keys alike."""
+        containing "cosine" switches on the query / key normalisation (:171-172,181-184), for raw and PQ-decoded keys alike.
+        searcher: a knn_search.KNNSearcher with the same k, used by get_knns when neither pending nor precomputed results exist."""
         assert metric_type in ["do_not_recomp_l2", "do_not_recomp_ip", "l2", "ip"]
         self.recompute = metric_type in ("l2", "ip")
         if self.recompute and keys is None and pq_codes is None:
@@ -42,6 +44,9 @@ class KNNModel(object):
         self.metric_type = metric_type
         self.k = k
         self.dists, self.knns = dists, knns
+        if searcher is not None and searcher.k != k:
+            raise ValueError(f"the searcher returns {searcher.k} neighbours, the model uses k = {k}")
+        self.searcher = searcher
         self._pending = None
 
     @property
@@ -71,7 +76,7 @@ class KNNModel(object):
                                cosine=self.cosine)
 
     def set_search_results(self, dists: Optional[torch.Tensor], knns: torch.Tensor):
-        """Provide the (out-of-scope) search output for the next get_knn_prob call: [num, k] each; dists may be None
+        """Provide the search output for the next get_knn_prob call: [num, k] each; dists may be None
         when the metric recomputes them."""
         self._pending = (None if dists is None else dists.contiguous().float(), knns.contiguous().long())
 
@@ -83,7 +88,9 @@ class KNNModel(object):
             positions = positions.reshape(-1)          # sample['positions'] is [B, L]: one row of search results per token
             return (None if self.dists is None else self.dists[positions].float().contiguous()), \
                 self.knns[positions].long().contiguous()
-        raise RuntimeError("faiss search is out of scope: call set_search_results() or pass precomputed arrays")
+        if self.searcher is not None:
+            return self.searcher.search(queries)
+        raise RuntimeError("no search results: pass a searcher, call set_search_results() or pass precomputed arrays")
 
     @torch.no_grad()
     def get_knn_prob(self, queries, k: int = 0, output_size: int = None, return_knn: bool = False, t: float = 1.0,

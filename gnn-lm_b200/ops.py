@@ -262,12 +262,14 @@ def split_tf32(w):
     return hi, lo
 
 
-def split_f16(w):
-    """fp32 [N, K] -> (fp16 hi, fp16 lo, power-of-two scale) for MATH_F16X3."""
+def split_f16(w, scale: Optional[float] = None):
+    """fp32 [N, K] -> (fp16 hi, fp16 lo, power-of-two scale) for MATH_F16X3; `scale` given: that one instead of the one that
+    brings max|w| to 2^13."""
     import math
     w = w.contiguous()
-    amax = float(w.abs().max().item()) if w.numel() else 1.0
-    scale = 2.0 ** math.floor(math.log2(8192.0 / amax)) if amax > 0 else 1.0
+    if scale is None:
+        amax = float(w.abs().max().item()) if w.numel() else 1.0
+        scale = 2.0 ** math.floor(math.log2(8192.0 / amax)) if amax > 0 else 1.0
     hi = torch.empty(w.shape, device=w.device, dtype=torch.float16)
     lo = torch.empty(w.shape, device=w.device, dtype=torch.float16)
     L.call("gnnlm_split_f16", L.ptr(w), float(scale), L.ptr(hi), L.ptr(lo), w.numel(), L.stream_ptr())
@@ -582,3 +584,37 @@ def knn_sims_pq(queries, rotated, codes, centroids, bias, ids, metric: str, *, k
            L.ptr(codes), codes.shape[0], M, dsub, L.ptr(centroids), L.ptr(bias), L.ptr(ids), ids.shape[1], METRICS[metric],
            L.ptr(key_norm2), (3 if metric == "ip" else 2) if cosine else 0, L.ptr(sims), T, L.stream_ptr())
     return sims
+
+
+def knn_filter(keys: Split, id_base: int, q_hi, q_lo, key_bias, thr, cand_s, cand_id, cand_cnt):
+    """Top-k filter pass of the exact kNN search over one span of keys (gnnlm_knn_filter_f16x3): appends (score, id) of every
+    score above thr[q] to cand_s / cand_id [n_q, cap] and counts it in cand_cnt (counts past cap flag an overflow)."""
+    n_q, d = q_hi.shape
+    assert keys.has_lo and keys.d == d and q_lo.shape == q_hi.shape and q_hi.stride(0) == q_lo.stride(0)
+    cap = cand_s.shape[1]
+    L.call("gnnlm_knn_filter_f16x3", L.ptr(keys.data), keys.data.stride(0), keys.data.shape[0], int(id_base), L.ptr(q_hi),
+           L.ptr(q_lo), q_hi.stride(0), n_q, d, L.ptr(key_bias), L.ptr(thr), L.ptr(cand_s), L.ptr(cand_id), L.ptr(cand_cnt), cap,
+           L.stream_ptr(), tag="knn_filter", work=(keys.data.shape[0], n_q, d))
+
+
+def topk_merge(top_s, top_id, cand_s, cand_id, cand_cnt, thr):
+    """Running top-k [n_q, k] (+) a span's candidates, in place; new thresholds; counts reset except for overflowed queries."""
+    n_q, k = top_s.shape
+    L.call("gnnlm_topk_merge", L.ptr(top_s), L.ptr(top_id), n_q, k, L.ptr(cand_s), L.ptr(cand_id), L.ptr(cand_cnt),
+           cand_s.shape[1], L.ptr(thr), L.stream_ptr(), tag="topk_merge")
+
+
+def knn_key_bias(x):
+    """-1/2 ||x_i||^2 [n] fp32 of fp16 / fp32 rows."""
+    assert x.dim() == 2 and x.stride(1) == 1
+    out = torch.empty((x.shape[0],), device=x.device, dtype=torch.float32)
+    L.call("gnnlm_knn_key_bias", L.ptr(x), L.dtype_code(x.dtype), x.stride(0), x.shape[0], x.shape[1], L.ptr(out), L.stream_ptr())
+    return out
+
+
+def knn_key_bias_pq(codes, norm2):
+    """-1/2 ||x_i||^2 [n] of PQ-decoded keys: codes [n, M] uint8, norm2 [M, 256] = ||centroid - b_m||^2."""
+    assert codes.dtype == torch.uint8 and codes.is_contiguous() and norm2.shape == (codes.shape[1], 256) and norm2.is_contiguous()
+    out = torch.empty((codes.shape[0],), device=codes.device, dtype=torch.float32)
+    L.call("gnnlm_knn_key_bias_pq", L.ptr(codes), codes.shape[0], codes.shape[1], L.ptr(norm2), L.ptr(out), L.stream_ptr())
+    return out

@@ -583,6 +583,31 @@ int32_t gnnlm_axpy_f32(float* y, int64_t ldy, const float* x, int64_t ldx, int64
 int32_t gnnlm_scatter_add_rows(float* dst, int64_t ld_dst, const float* src, int64_t ld_src, const int32_t* ids, int64_t rows,
                                const int32_t* rows_dev, int64_t cols, gnnlm_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * (10) Exact k-nearest-neighbour search over the datastore -- replaces the faiss index search that writes the neighbour-id files
+ *      (knn/find_knn.py:29-71) and KNNModel.get_knns (knn/knn_model.py:87-101).  For every query q the k rows x with the highest
+ *      score s(q, x) = q.x + bias(x), ties by smaller id; bias = -1/2 ||x||^2 ranks like squared L2 (faiss METRIC_L2), bias = 0 is
+ *      inner product.  The datastore is scanned in spans of increasing ids; per span:
+ *
+ * gnnlm_knn_filter_f16x3: the 3xFP16 tcgen05 product of the span's keys [n_keys, 2d] (split fp16, GNNLM_F16X2, ldk >= 2d; row r has
+ *   id id_base + r, id_base + n_keys < 2^31) with the queries q_hi / q_lo [n_q, d] fp16 (gnnlm_split_f16 with scale 1, ldq >= d),
+ *   plus key_bias [n_keys] fp32 (nullable = 0).  Nothing per (key, query) is stored: a score with s > thr[q] is appended to
+ *   cand_s / cand_id [n_q, cap] (order within a span unspecified) and counted in cand_cnt[q] (zero it before the first span).  Past cap
+ *   the writes stop and the count keeps growing: cand_cnt[q] > cap flags an overflowed query.  1 <= cap <= 4096, d % 8 == 0.
+ * gnnlm_topk_merge: per query, merge the running top_s / top_id [n_q, k] (sorted, id -1 = empty, score -inf) with its min(cnt, cap)
+ *   candidates into the new sorted top-k, write thr[q] = its k-th score (-inf while fewer than k are held) and reset cand_cnt[q]
+ *   to 0.  Queries with cand_cnt[q] > cap are left untouched (count included).  1 <= k <= 2048, 1 <= cap <= 4096.  Deterministic.
+ * gnnlm_knn_key_bias: out[i] = -1/2 ||x_i||^2 (fp32, fixed summation order) of fp32 / fp16 rows x [n, d] (ld elements).
+ * gnnlm_knn_key_bias_pq: the same for PQ-decoded keys: out[i] = -1/2 sum_m norm2[m, codes[i, m]], norm2 [M, 256] fp32 =
+ *   ||centroid[m, c] - b_m||^2, codes [n, M] uint8. */
+int32_t gnnlm_knn_filter_f16x3(const void* keys, int64_t ldk, int64_t n_keys, int64_t id_base, const void* q_hi, const void* q_lo,
+                               int64_t ldq, int64_t n_q, int64_t d, const float* key_bias, const float* thr, float* cand_s,
+                               int32_t* cand_id, int32_t* cand_cnt, int64_t cap, gnnlm_stream_t stream);
+int32_t gnnlm_topk_merge(float* top_s, int32_t* top_id, int64_t n_q, int32_t k, const float* cand_s, const int32_t* cand_id,
+                         int32_t* cand_cnt, int64_t cap, float* thr, gnnlm_stream_t stream);
+int32_t gnnlm_knn_key_bias(const void* x, int32_t dtype, int64_t ld, int64_t n, int64_t d, float* out, gnnlm_stream_t stream);
+int32_t gnnlm_knn_key_bias_pq(const uint8_t* codes, int64_t n, int32_t M, const float* norm2, float* out, gnnlm_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
