@@ -52,6 +52,8 @@ SIGNATURES = {
     "gnnlm_quant_w8": (_i32, [_p, _p, _i64, _p, _i64, _i64, _i64, _p]),
     "gnnlm_linear_f16f8": (_i32, [_p, _p, _i64, _i64, _i64, _p, _p, _i64, _i64, _i64, _p, _p, _f32, _i64, _i64, _p, _p, _i32, _i64,
                                   _i64, _p, _i64, _p, _p]),
+    "gnnlm_linear_f16f8_nn_attn": (_i32, [_p, _p, _i64, _i64, _i64, _p, _p, _f32, _i64, _i64, _p, _p, _p, _i32, _i32, _p, _i64, _p,
+                                          _i64, _p, _i64, _p, _p]),
     "gnnlm_lse_num_tiles": (_i64, [_i64, _i32]),
     "gnnlm_linear_lse": (_i32, [_p, _i32, _i64, _p, _p, _f32, _i64, _p, _p, _p, _p, _i64, _p, _i64, _i64, _i32, _p]),
     "gnnlm_lse_finish": (_i32, [_p, _p, _p, _i64, _p, _p, _i32, _i64, _p, _p]),

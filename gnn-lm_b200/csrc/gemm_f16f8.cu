@@ -52,9 +52,186 @@ struct F8Maps {
   CUtensorMap wh, w8_lo, w8_hi;         // W fp16 hi (scaled), e4m3 lo8 / hi8
 };
 
+// Chain attention of the ntgt-intra-ntgt edges fused into the epilogue of the head-interleaved Q | K' | V' projection
+// (gnnlm_linear_f16f8_nn_attn).  W rows are [Q_0 | K'_0 | Q_1 | K'_1 | ... | V'_0 .. V'_{H-1}] with d_k = 128, so N-tile h < H holds
+// head h's Q and K' and N-tile H + j the V' of heads 2j, 2j + 1.  A CTA pair runs all 3H / 2 N-tiles of its two row windows in
+// that order: the QK tiles leave the softmax weights alpha (3 per head: left / self / right chain neighbour) in registers, the V
+// tiles mix the neighbours' V' rows and write the A-linear operand; Q | K' | V' never reach memory.
+// Window j covers rows [j S - h, j S - h + 128) and owns [j S, j S + S), S = 128 - 2h, h = w - 1: a chain neighbour is at
+// most h ids away, so every neighbour of an owned row is a lane of the same accumulator.
+struct NnAttn {
+  const int32_t* indptr;     // nn_indptr / nn_indices: [left,] self[, right] per row, in chain order
+  const int32_t* indices;
+  __half* out;               // [M, ld_out] fp16 hi of the attention output
+  int64_t ld_out;
+  uint8_t* q8;               // [M, ldq8] its e4m3 companion: hi8 at column c, lo8 at column d + c (no fp16 lo half)
+  int64_t ldq8;
+  int32_t* err;              // set to 1 when an owned row has a neighbour outside its window or more than three edges
+  int halo;                  // h
+  int heads;                 // H
+};
+constexpr int NN_BAR = 1;                                   // named barrier of the four epilogue warps (fused attention only)
+
+__device__ __forceinline__ void nn_bar() { asm volatile("bar.sync %0, %1;" ::"r"(NN_BAR), "r"(4 * 32) : "memory"); }
+
+// One window row per thread (TMEM lane L).  Per 32-column chunk every thread stages its K' (or V') row in the CTA-wide tile, and
+// reads its neighbours' rows back: the rows of the warp's edges are other warps' lanes.  Rows a window does not own, and rows
+// >= M, run the same instructions with themselves as their only neighbour and store nothing, so that every thread reaches every
+// barrier equally often.  The arithmetic follows cluster_attn_kernel: same scores up to the summation order of the dot products,
+// same softmax and mixing order.
+template <class TileRC>
+__device__ __forceinline__ void nn_attn_epilogue(uint32_t tmem_base, int64_t pair0, int64_t pair_stride, int64_t total, int64_t n_p,
+                                                 int64_t M, int S, uint32_t crank, int q, const float* __restrict__ bias,
+                                                 float acc_scale, const NnAttn& na, float* tile, uint64_t* tmem_full,
+                                                 uint64_t* tmem_empty, TileRC tile_rc) {
+  const int lane = threadIdx.x & 31;
+  const int L = q * 32 + lane;
+  const uint32_t my_row = smem_u32(tile + L * EPI_LD);
+  const int H = na.heads, d = H * 128;
+  float al[8], as[8], ar[8];                                // alpha of the left / self / right neighbour, per head
+#pragma unroll
+  for (int h = 0; h < 8; ++h) al[h] = as[h] = ar[h] = 0.f;
+  int ll = L, lr = L;                                       // neighbour lanes (own lane: no such neighbour)
+  bool own = false;
+  int64_t g = 0;
+  int64_t it = 0;
+  for (int64_t t = pair0; t < total; t += pair_stride, ++it) {
+    int64_t r, c;
+    tile_rc(t, r, c);
+    if (r >= n_p) break;
+    if (c == 0) {                                           // first tile of a window
+      const int64_t g0 = (r * 2 + crank) * S - na.halo;
+      g = g0 + L;
+      own = L >= na.halo && L < na.halo + S && g < M;
+      ll = lr = L;
+      if (own) {
+        const int e0 = __ldg(na.indptr + g), deg = __ldg(na.indptr + g + 1) - e0;
+        int64_t ml = g, mr = g;
+        if (deg == 3) {
+          ml = __ldg(na.indices + e0);
+          mr = __ldg(na.indices + e0 + 2);
+        } else if (deg == 2) {
+          const int64_t a = __ldg(na.indices + e0);
+          if (a == g) mr = __ldg(na.indices + e0 + 1);
+          else ml = a;
+        }
+        const int64_t dl = ml - g0, dr = mr - g0;
+        if (deg < 1 || deg > 3 || dl < 0 || dl >= BLOCK_M || dr < 0 || dr >= BLOCK_M) {
+          *na.err = 1;
+        } else {
+          ll = (int)dl;
+          lr = (int)dr;
+        }
+      }
+    }
+    const uint32_t rl = smem_u32(tile + ll * EPI_LD), rr = smem_u32(tile + lr * EPI_LD);
+    const int acc = (int)(it & 1);
+    const uint32_t acc_phase = (uint32_t)((it >> 1) & 1);
+    mbar_wait(&tmem_full[acc], acc_phase);
+    tc_fence_after();
+    __syncwarp();                                           // the tcgen05.ld below are warp-collective
+    const uint32_t taddr = tmem_base + (uint32_t)acc * BLOCK_N + ((uint32_t)(q * 32) << 16);
+    const float* bt = bias + c * BLOCK_N;
+    if (c < H) {                                            // head c: Q in columns [0, 128), K' in [128, 256)
+      float s_l = 0.f, s_s = 0.f, s_r = 0.f;
+#pragma unroll 1
+      for (int cc = 0; cc < 128; cc += 32) {
+        float qv[32], kv[32];
+        tmem_ld32_issue(taddr + (uint32_t)cc, qv);
+        tmem_ld32_issue(taddr + (uint32_t)(128 + cc), kv);
+        tmem_ld_wait(qv);
+        tmem_ld_wait(kv);
+#pragma unroll
+        for (int j = 0; j < 32; j += 4) {
+          const float4 bq = __ldg(reinterpret_cast<const float4*>(bt + cc + j));
+          const float4 bk = __ldg(reinterpret_cast<const float4*>(bt + 128 + cc + j));
+          qv[j] = fmaf(qv[j], acc_scale, bq.x); qv[j + 1] = fmaf(qv[j + 1], acc_scale, bq.y);
+          qv[j + 2] = fmaf(qv[j + 2], acc_scale, bq.z); qv[j + 3] = fmaf(qv[j + 3], acc_scale, bq.w);
+          kv[j] = fmaf(kv[j], acc_scale, bk.x); kv[j + 1] = fmaf(kv[j + 1], acc_scale, bk.y);
+          kv[j + 2] = fmaf(kv[j + 2], acc_scale, bk.z); kv[j + 3] = fmaf(kv[j + 3], acc_scale, bk.w);
+          sts128(my_row + 4 * j, kv[j], kv[j + 1], kv[j + 2], kv[j + 3]);
+        }
+        nn_bar();
+#pragma unroll
+        for (int j = 0; j < 32; j += 4) {
+          const float4 a = lds128(rl + 4 * j), b = lds128(rr + 4 * j);
+          s_s = fmaf(qv[j], kv[j], s_s); s_s = fmaf(qv[j + 1], kv[j + 1], s_s);
+          s_s = fmaf(qv[j + 2], kv[j + 2], s_s); s_s = fmaf(qv[j + 3], kv[j + 3], s_s);
+          s_l = fmaf(qv[j], a.x, s_l); s_l = fmaf(qv[j + 1], a.y, s_l); s_l = fmaf(qv[j + 2], a.z, s_l); s_l = fmaf(qv[j + 3], a.w, s_l);
+          s_r = fmaf(qv[j], b.x, s_r); s_r = fmaf(qv[j + 1], b.y, s_r); s_r = fmaf(qv[j + 2], b.z, s_r); s_r = fmaf(qv[j + 3], b.w, s_r);
+        }
+        nn_bar();
+      }
+      if (ll == L) s_l = -INFINITY;
+      if (lr == L) s_r = -INFINITY;
+      const float mx = fmaxf(s_s, fmaxf(s_l, s_r));
+      const float e0 = __expf(s_l - mx), e1 = __expf(s_s - mx), e2 = __expf(s_r - mx);
+      const float inv = __fdividef(1.f, e0 + e1 + e2);
+#pragma unroll
+      for (int h = 0; h < 8; ++h)
+        if (h == c) { al[h] = e0 * inv; as[h] = e1 * inv; ar[h] = e2 * inv; }
+    } else {                                                // V' of heads 2 (c - H) and 2 (c - H) + 1
+      const int64_t col0 = (c - H) * BLOCK_N;
+#pragma unroll 1
+      for (int cc = 0; cc < BLOCK_N; cc += 32) {
+        const int hd = (int)(2 * (c - H)) + (cc >= 128 ? 1 : 0);
+        float wl = 0.f, ws = 0.f, wr = 0.f;
+#pragma unroll
+        for (int h = 0; h < 8; ++h)
+          if (h == hd) { wl = al[h]; ws = as[h]; wr = ar[h]; }
+        float v[32];
+        tmem_ld32(taddr + (uint32_t)cc, v);
+#pragma unroll
+        for (int j = 0; j < 32; j += 4) {
+          const float4 bv = __ldg(reinterpret_cast<const float4*>(bt + cc + j));
+          v[j] = fmaf(v[j], acc_scale, bv.x); v[j + 1] = fmaf(v[j + 1], acc_scale, bv.y);
+          v[j + 2] = fmaf(v[j + 2], acc_scale, bv.z); v[j + 3] = fmaf(v[j + 3], acc_scale, bv.w);
+          sts128(my_row + 4 * j, v[j], v[j + 1], v[j + 2], v[j + 3]);
+        }
+        nn_bar();
+#pragma unroll
+        for (int j = 0; j < 32; j += 4) {
+          const float4 a = lds128(rl + 4 * j), b = lds128(rr + 4 * j);
+          v[j] = fmaf(wr, b.x, fmaf(wl, a.x, ws * v[j]));
+          v[j + 1] = fmaf(wr, b.y, fmaf(wl, a.y, ws * v[j + 1]));
+          v[j + 2] = fmaf(wr, b.z, fmaf(wl, a.z, ws * v[j + 2]));
+          v[j + 3] = fmaf(wr, b.w, fmaf(wl, a.w, ws * v[j + 3]));
+        }
+        nn_bar();
+        if (own) {                                          // 64 B of fp16 hi + 2 x 32 B of e4m3: whole sectors per row
+          uint32_t hi[16], h8[8], l8[8];
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            uint2 h2, l2;
+            split4_f16(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3], h2, l2);
+            q8_from_split4(h2, l2, h8[i], l8[i]);
+            hi[2 * i] = h2.x;
+            hi[2 * i + 1] = h2.y;
+          }
+          uint4* op = reinterpret_cast<uint4*>(na.out + g * na.ld_out + col0 + cc);
+          uint4* qh = reinterpret_cast<uint4*>(na.q8 + g * na.ldq8 + col0 + cc);
+          uint4* ql = reinterpret_cast<uint4*>(na.q8 + g * na.ldq8 + d + col0 + cc);
+#pragma unroll
+          for (int i = 0; i < 4; ++i) op[i] = make_uint4(hi[4 * i], hi[4 * i + 1], hi[4 * i + 2], hi[4 * i + 3]);
+#pragma unroll
+          for (int i = 0; i < 2; ++i) {
+            qh[i] = make_uint4(h8[4 * i], h8[4 * i + 1], h8[4 * i + 2], h8[4 * i + 3]);
+            ql[i] = make_uint4(l8[4 * i], l8[4 * i + 1], l8[4 * i + 2], l8[4 * i + 3]);
+          }
+        }
+        __syncwarp();                                       // reconverge before the next chunk's tcgen05.ld and bar.sync
+      }
+    }
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) mbar_arrive_leader(&tmem_empty[acc]);
+  }
+}
+
+template <bool NN>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
     gemm_f16f8_kernel(const __grid_constant__ F8Maps maps, int64_t M_cap, const int32_t* __restrict__ m_dev, int64_t N, int64_t K,
-                      int kb_split, EpiStore es, float acc_scale, int dbg, long long* __restrict__ dbg_out) {
+                      int kb_split, EpiStore es, float acc_scale, int dbg, long long* __restrict__ dbg_out, NnAttn na) {
   constexpr int STAGES = F8_STAGES;
   constexpr uint32_t TX = 2u * F8_STAGE;                                  // both CTAs' six operand tiles -> leader
   const int n_mma = N <= BLOCK_N / 2 ? BLOCK_N / 2 : BLOCK_N;
@@ -72,10 +249,24 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
   const uint32_t crank = cluster_ctarank();
   const bool leader = crank == 0;
   const int64_t M = live_rows(M_cap, m_dev);
-  const int64_t n_m = (M + BLOCK_M - 1) / BLOCK_M, n_n = (N + BLOCK_N - 1) / BLOCK_N;
-  const int64_t n_p = (n_m + 1) / 2;
-  const int64_t total = n_p * n_n;
   const int64_t pair0 = blockIdx.x >> 1, pair_stride = gridDim.x >> 1;
+  // NN: row blocks are windows of S owned rows, and a pair takes all n_n N-tiles of its windows before moving on
+  const int S = NN ? BLOCK_M - 2 * na.halo : BLOCK_M;
+  const int64_t n_m = (M + S - 1) / S, n_n = (N + BLOCK_N - 1) / BLOCK_N;
+  const int64_t n_p = (n_m + 1) / 2;
+  const int64_t total = NN ? (n_p + pair_stride - 1) / pair_stride * pair_stride * n_n : n_p * n_n;
+  // (pair row block r, N-tile c) of a tile index; every role walks the same sequence and stops at r >= n_p
+  auto tile_rc = [&](int64_t tile, int64_t& r, int64_t& c) {
+    if (NN) {
+      const int64_t k = tile / pair_stride;
+      r = tile % pair_stride + k / n_n * pair_stride;
+      c = k % n_n;
+    } else {
+      r = tile / n_n;
+      c = tile % n_n;
+    }
+  };
+  auto row0 = [&](int64_t r) { return (r * 2 + crank) * S - (NN ? na.halo : 0); };     // first A row of this CTA's block
   const int n_kb = (int)((K + F8_BLOCK_K - 1) / F8_BLOCK_K);
 
   auto sAh = [&](int s) { return smem + (size_t)s * F8_STAGE; };
@@ -120,8 +311,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
       const int half = (int)crank * (n_mma / 2);
       long long t_wait = 0;
       for (int64_t tile = pair0; tile < total; tile += pair_stride) {
-        const int64_t r = tile / n_n, c = tile % n_n;
-        const int m0 = (int)((r * 2 + crank) * BLOCK_M), n0 = (int)(c * BLOCK_N) + half;
+        int64_t r, c;
+        tile_rc(tile, r, c);
+        if (r >= n_p) break;
+        const int m0 = (int)row0(r), n0 = (int)(c * BLOCK_N) + half;      // NN, window 0: m0 = -h, zero-filled by TMA
         for (int kb = 0; kb < n_kb; ++kb) {
           const long long t0 = dbg_out ? clock64() : 0;
           mbar_wait(&empty_bar[stage], phase ^ 1);
@@ -148,6 +341,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
       long long t_empty = 0, t_full = 0;
       const long long t_begin = dbg_out ? clock64() : 0;
       for (int64_t tile = pair0; tile < total; tile += pair_stride, ++it) {
+        if (NN) {
+          int64_t r, c;
+          tile_rc(tile, r, c);
+          if (r >= n_p) break;
+        }
         const int acc = (int)(it & 1);
         const uint32_t acc_phase = (uint32_t)((it >> 1) & 1);
         const long long te0 = dbg_out ? clock64() : 0;
@@ -188,6 +386,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
     }
   } else if (warp >= EPI_WARP0 && warp < EPI_WARP0 + EPI_WARPS) {
     const int q = warp & 3;                            // ---- epilogue (both CTAs)
+    if constexpr (NN) {
+      nn_attn_epilogue(tmem_base, pair0, pair_stride, total, n_p, M, S, crank, q, es.bias, acc_scale, na, epi_smem,
+                       tmem_full, tmem_empty, tile_rc);
+    } else {
     int64_t it = 0;
     EpiLse el{};
     long long t_epi_wait = 0, t_epi_work = 0;
@@ -211,6 +413,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
     if (dbg_out && lane == 0) {
       dbg_out[blockIdx.x * 8 + 4 + (q & 1) * 2] = t_epi_wait;       // warps 0 / 1 of the four (2 / 3 overwrite: same order of magnitude)
       dbg_out[blockIdx.x * 8 + 5 + (q & 1) * 2] = t_epi_work;
+    }
     }
   }
 
@@ -314,30 +517,22 @@ extern "C" int32_t gnnlm_quant_w8(const void* w_hi, const void* w_lo, int64_t ld
   return 0;
 }
 
-extern "C" int32_t gnnlm_linear_f16f8(const void* A1, const void* A1q, int64_t lda1, int64_t ldq1, int64_t K1, const void* A2,
-                                      const void* A2q, int64_t lda2, int64_t ldq2, int64_t K2, const void* W_hi, const void* W8,
-                                      float w_scale, int64_t ldw, int64_t ldw8, const float* bias, void* C, int32_t c_dtype,
-                                      int64_t ldc, int64_t M, const int32_t* m_dev, int64_t N, void* C8, cudaStream_t stream) {
-  GNNLM_CHECK_ARG(A1 && A1q && W_hi && W8 && C && M >= 0 && N > 0 && K1 > 0 && K2 >= 0 && w_scale > 0.f, GNNLM_E_ARG,
-                  "gnnlm_linear_f16f8: null pointer / bad sizes");
-  GNNLM_CHECK_ARG(K2 == 0 || (A2 && A2q), GNNLM_E_ARG, "gnnlm_linear_f16f8: K2 > 0 needs the second source");
-  GNNLM_CHECK_ARG(c_dtype == GNNLM_F32 || c_dtype == GNNLM_BF16 || c_dtype == GNNLM_F16X2 || c_dtype == GNNLM_F24, GNNLM_E_ARG,
-                  "gnnlm_linear_f16f8: output dtype must be f32 / bf16 / split fp16 / f24");
-  GNNLM_CHECK_ARG(c_dtype != GNNLM_F24 || (C8 && N % 4 == 0 && ldc % 4 == 0 && (uintptr_t)C % 16 == 0 && (uintptr_t)C8 % 4 == 0),
-                  GNNLM_E_SHAPE, "gnnlm_linear_f16f8: GNNLM_F24 output needs the byte plane, N and ldc multiples of 4, aligned bases");
-  GNNLM_CHECK_ARG(gemm_tc_supported(), GNNLM_E_UNSUPPORTED, "gnnlm_linear_f16f8: needs an sm_100 device and driver TMA support");
+// operand checks and tensor maps shared by gnnlm_linear_f16f8 and gnnlm_linear_f16f8_nn_attn
+static int32_t f8_maps(const char* who, tc::F8Maps& maps, const void* A1, const void* A1q, int64_t lda1, int64_t ldq1, int64_t K1,
+                       const void* A2, const void* A2q, int64_t lda2, int64_t ldq2, int64_t K2, const void* W_hi, const void* W8,
+                       int64_t ldw, int64_t ldw8, int64_t M, int64_t N) {
+  GNNLM_CHECK_ARG(gemm_tc_supported(), GNNLM_E_UNSUPPORTED, "%s: needs an sm_100 device and driver TMA support", who);
   const int64_t K = K1 + K2;
   // k-blocks of 64 must not straddle the two sources; e4m3 halves sit K1 (resp. K2, K) bytes apart inside their rows
   GNNLM_CHECK_ARG(K1 % tc::F8_BLOCK_K == 0 && K2 % 16 == 0 && K1 % 16 == 0 && lda1 >= K1 && ldq1 >= 2 * K1 && ldw >= K &&
                       ldw8 >= 2 * K && (K2 == 0 || (lda2 >= K2 && ldq2 >= 2 * K2)),
-                  GNNLM_E_SHAPE, "gnnlm_linear_f16f8: K1 must be a multiple of 64, K1 / K2 multiples of 16 (K1=%lld K2=%lld)",
-                  (long long)K1, (long long)K2);
+                  GNNLM_E_SHAPE, "%s: K1 must be a multiple of 64, K1 / K2 multiples of 16 (K1=%lld K2=%lld)",
+                  who, (long long)K1, (long long)K2);
   GNNLM_CHECK_ARG((lda1 * 2) % 16 == 0 && ldq1 % 16 == 0 && (ldw * 2) % 16 == 0 && ldw8 % 16 == 0 && (uintptr_t)A1 % 16 == 0 &&
                       (uintptr_t)A1q % 16 == 0 && (uintptr_t)W_hi % 16 == 0 && (uintptr_t)W8 % 16 == 0 &&
                       (K2 == 0 || ((lda2 * 2) % 16 == 0 && ldq2 % 16 == 0 && (uintptr_t)A2 % 16 == 0 && (uintptr_t)A2q % 16 == 0)),
-                  GNNLM_E_SHAPE, "gnnlm_linear_f16f8: TMA needs 16 B aligned bases and row strides");
+                  GNNLM_E_SHAPE, "%s: TMA needs 16 B aligned bases and row strides", who);
   if (M == 0) return 0;
-  tc::F8Maps maps;
   const uint8_t* a1q = reinterpret_cast<const uint8_t*>(A1q);
   const uint8_t* w8 = reinterpret_cast<const uint8_t*>(W8);
   int r = tc::make_map_k64(&maps.a1h, A1, 2, M, K1, lda1 * 2, tc::BLOCK_M);
@@ -356,14 +551,33 @@ extern "C" int32_t gnnlm_linear_f16f8(const void* A1, const void* A1q, int64_t l
   if (!r) r = tc::make_map_k64(&maps.wh, W_hi, 2, N, K, ldw * 2, tc::BLOCK_N / 2);
   if (!r) r = tc::make_map_k64(&maps.w8_lo, w8, 1, N, K, ldw8, tc::BLOCK_N / 2);
   if (!r) r = tc::make_map_k64(&maps.w8_hi, w8 + K, 1, N, K, ldw8, tc::BLOCK_N / 2);
-  GNNLM_CHECK_ARG(r == 0, GNNLM_E_ARG, "gnnlm_linear_f16f8: cuTensorMapEncodeTiled failed (%d)", r);
+  GNNLM_CHECK_ARG(r == 0, GNNLM_E_ARG, "%s: cuTensorMapEncodeTiled failed (%d)", who, r);
+  return 0;
+}
+
+extern "C" int32_t gnnlm_linear_f16f8(const void* A1, const void* A1q, int64_t lda1, int64_t ldq1, int64_t K1, const void* A2,
+                                      const void* A2q, int64_t lda2, int64_t ldq2, int64_t K2, const void* W_hi, const void* W8,
+                                      float w_scale, int64_t ldw, int64_t ldw8, const float* bias, void* C, int32_t c_dtype,
+                                      int64_t ldc, int64_t M, const int32_t* m_dev, int64_t N, void* C8, cudaStream_t stream) {
+  GNNLM_CHECK_ARG(A1 && A1q && W_hi && W8 && C && M >= 0 && N > 0 && K1 > 0 && K2 >= 0 && w_scale > 0.f, GNNLM_E_ARG,
+                  "gnnlm_linear_f16f8: null pointer / bad sizes");
+  GNNLM_CHECK_ARG(K2 == 0 || (A2 && A2q), GNNLM_E_ARG, "gnnlm_linear_f16f8: K2 > 0 needs the second source");
+  GNNLM_CHECK_ARG(c_dtype == GNNLM_F32 || c_dtype == GNNLM_BF16 || c_dtype == GNNLM_F16X2 || c_dtype == GNNLM_F24, GNNLM_E_ARG,
+                  "gnnlm_linear_f16f8: output dtype must be f32 / bf16 / split fp16 / f24");
+  GNNLM_CHECK_ARG(c_dtype != GNNLM_F24 || (C8 && N % 4 == 0 && ldc % 4 == 0 && (uintptr_t)C % 16 == 0 && (uintptr_t)C8 % 4 == 0),
+                  GNNLM_E_SHAPE, "gnnlm_linear_f16f8: GNNLM_F24 output needs the byte plane, N and ldc multiples of 4, aligned bases");
+  tc::F8Maps maps;
+  if (int32_t rc = f8_maps("gnnlm_linear_f16f8", maps, A1, A1q, lda1, ldq1, K1, A2, A2q, lda2, ldq2, K2, W_hi, W8, ldw, ldw8, M, N))
+    return rc;
+  if (M == 0) return 0;
+  const int64_t K = K1 + K2;
 
   tc::EpiStore es{bias, nullptr, 0, C, ldc, c_dtype == GNNLM_BF16 ? 1 : (c_dtype == GNNLM_F16X2 ? 2 : (c_dtype == GNNLM_F24 ? 3 : 0)), 0, N, N};
   es.C8 = reinterpret_cast<uint8_t*>(C8);
   const size_t smem = (size_t)tc::F8_STAGES * tc::F8_STAGE + tc::EPI_SMEM + 1024;
   static bool attr_set = false;
   if (!attr_set) {
-    GNNLM_CUDA(cudaFuncSetAttribute(tc::gemm_f16f8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    GNNLM_CUDA(cudaFuncSetAttribute(tc::gemm_f16f8_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_set = true;
   }
   static int n_sm = 0;
@@ -387,7 +601,8 @@ extern "C" int32_t gnnlm_linear_f16f8(const void* A1, const void* A1q, int64_t l
     GNNLM_CUDA(cudaMemsetAsync(buf, 0, 148 * 8 * sizeof(long long), stream));
     dbg_out = buf;
   }
-  tc::gemm_f16f8_kernel<<<grid, 256, smem, stream>>>(maps, M, m_dev, N, K, (int)(K1 / tc::F8_BLOCK_K), es, 1.f / w_scale, dbg, dbg_out);
+  tc::gemm_f16f8_kernel<false><<<grid, 256, smem, stream>>>(maps, M, m_dev, N, K, (int)(K1 / tc::F8_BLOCK_K), es, 1.f / w_scale, dbg,
+                                                           dbg_out, tc::NnAttn{});
   GNNLM_LAUNCH_CHECK("gnnlm_linear_f16f8");
   if (dbg_out) {
     static long long host[148 * 8];
@@ -404,5 +619,44 @@ extern "C" int32_t gnnlm_linear_f16f8(const void* A1, const void* A1q, int64_t l
             "epi warp0 wait %.0f work %.0f, warp1 wait %.0f work %.0f\n", (long long)M, (long long)N, (long long)K, acc[3] / n_lead,
             acc[1] / n_lead, acc[2] / n_lead, acc[0] / grid, acc[4] / grid, acc[5] / grid, acc[6] / grid, acc[7] / grid);
   }
+  return 0;
+}
+
+extern "C" int32_t gnnlm_linear_f16f8_nn_attn(const void* A, const void* Aq, int64_t lda, int64_t ldq, int64_t K, const void* W_hi,
+                                              const void* W8, float w_scale, int64_t ldw, int64_t ldw8, const float* bias,
+                                              const int32_t* nn_indptr, const int32_t* nn_indices, int32_t max_cluster, int32_t H,
+                                              void* out, int64_t ldo, void* q8, int64_t ldq8, int32_t* err, int64_t M,
+                                              const int32_t* m_dev, cudaStream_t stream) {
+  GNNLM_CHECK_ARG(A && Aq && W_hi && W8 && bias && nn_indptr && nn_indices && out && q8 && err && M >= 0 && K > 0 && w_scale > 0.f,
+                  GNNLM_E_ARG, "gnnlm_linear_f16f8_nn_attn: null pointer / bad sizes");
+  GNNLM_CHECK_ARG((max_cluster == 1 || max_cluster == 3 || max_cluster == 5 || max_cluster == 7) && H >= 2 && H <= 8 && H % 2 == 0,
+                  GNNLM_E_UNSUPPORTED, "gnnlm_linear_f16f8_nn_attn: needs clusters of 1, 3, 5 or 7 nodes and an even H <= 8 (w=%d, H=%d)",
+                  max_cluster, H);
+  const int64_t d = (int64_t)H * 128, N = 3 * d;
+  GNNLM_CHECK_ARG(ldo >= d && ldo % 8 == 0 && ldq8 >= 2 * d && ldq8 % 16 == 0 && (uintptr_t)out % 16 == 0 && (uintptr_t)q8 % 16 == 0 &&
+                      (uintptr_t)bias % 16 == 0,
+                  GNNLM_E_SHAPE, "gnnlm_linear_f16f8_nn_attn: output rows / bias must be 16 B aligned, ldo >= d, ldq8 >= 2d");
+  tc::F8Maps maps;
+  if (int32_t rc = f8_maps("gnnlm_linear_f16f8_nn_attn", maps, A, Aq, lda, ldq, K, nullptr, nullptr, 0, 0, 0, W_hi, W8, ldw, ldw8, M, N))
+    return rc;
+  if (M == 0) return 0;
+  const int halo = max_cluster - 1, S = tc::BLOCK_M - 2 * halo;
+  tc::NnAttn na{nn_indptr, nn_indices, reinterpret_cast<__half*>(out), ldo, reinterpret_cast<uint8_t*>(q8), ldq8, err, halo, H};
+  tc::EpiStore es{bias, nullptr, 0, nullptr, 0, 0, 0, 0, 0};
+  const size_t smem = (size_t)tc::F8_STAGES * tc::F8_STAGE + tc::EPI_SMEM + 1024;
+  static bool attr_set[MAX_DEVICES] = {false};
+  const int slot = device_slot();
+  if (!attr_set[slot]) {
+    GNNLM_CUDA(cudaFuncSetAttribute(tc::gemm_f16f8_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attr_set[slot] = true;
+  }
+  int dev = 0, n_sm = 0;
+  GNNLM_CUDA(cudaGetDevice(&dev));
+  GNNLM_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
+  const int64_t pairs = ceil_div(ceil_div(M, S), 2);        // window pairs at capacity; the kernel walks those of the live M
+  const unsigned grid = 2u * (unsigned)(pairs < n_sm / 2 ? pairs : n_sm / 2);
+  tc::gemm_f16f8_kernel<true><<<grid, 256, smem, stream>>>(maps, M, m_dev, N, K, (int)(K / tc::F8_BLOCK_K), es, 1.f / w_scale, 0, nullptr,
+                                                          na);
+  GNNLM_LAUNCH_CHECK("gnnlm_linear_f16f8_nn_attn");
   return 0;
 }

@@ -68,6 +68,17 @@ class _Weight:
             self._q8 = ops.quant_w8(self.W, self.lo)
         return self._q8
 
+    def permuted(self, perm: torch.Tensor) -> "_Weight":
+        """The same prepared weight with its rows (and bias entries) in the order `perm`."""
+        v = object.__new__(_Weight)
+        v.f8 = self.f8
+        v._q8 = self.w8()[perm].contiguous() if self.f8 else None
+        v.W = self.W[perm].contiguous()
+        v.lo = None if self.lo is None else self.lo[perm].contiguous()
+        v.b = None if self.b is None else self.b[perm].contiguous()
+        v.scale = self.scale
+        return v
+
     def rows(self, a: int, b_: int) -> "_Weight":
         v = object.__new__(_Weight)
         v.f8 = self.f8
@@ -77,6 +88,15 @@ class _Weight:
         v.b = None if self.b is None else self.b[a:b_]
         v.scale = self.scale
         return v
+
+
+def head_interleave(H: int, dk: int) -> torch.Tensor:
+    """Row order [Q_0 | K'_0 | Q_1 | K'_1 | ... | Q_{H-1} | K'_{H-1} | V'_0 .. V'_{H-1}] of a [Q | K' | V'] projection: with d_k = 128
+    every 256-row tile of the first 2 d rows holds one head's Q and K', every one of the last d rows the V' of two heads
+    (the N-tiles of gnnlm_linear_f16f8_nn_attn)."""
+    d = H * dk
+    qk = torch.arange(d).view(H, dk)
+    return torch.cat([torch.stack([qk, qk + d], 1).reshape(-1), torch.arange(2 * d, 3 * d)])
 
 
 FUSED_INTER_MODES = (L.MATH_F16X3, L.MATH_F16F8, L.MATH_BF16, L.MATH_TF32)     # modes whose operands are already fp16-range on tensor cores
@@ -193,6 +213,8 @@ class HGTLayer(hetero.IncrementalState, nn.Module):
         self.use_hq_attention = {"0": False, "all": "all"}.get(os.environ.get("GNNLM_HQ", "1"), True)
         # layer 0 with the rotation folded, followed by the centre-only layer: LayerNorm deferred into its consumers (HGT._ntgt_side)
         self.use_deferred_ln = os.environ.get("GNNLM_DEFER_LN", "1") != "0"
+        # MATH_F16F8, d_k = 128: the all-nodes chain attention in the epilogue of its Q|K'|V' projection (GNNLM_FUSED_NN=0: two kernels, for A/B)
+        self.use_fused_nn = os.environ.get("GNNLM_FUSED_NN", "1") != "0"
 
     # ------------------------------------------------------------------ weight preparation
     def prepare(self, math_mode: int, rot: Optional[torch.Tensor] = None, prev_ln=None):
@@ -250,6 +272,9 @@ class HGTLayer(hetero.IncrementalState, nn.Module):
             "a_rot": None if rot is None else _Weight(torch.cat([self.a_linears[n].weight.detach().float(), rot.detach().float()], 1),
                                                       self.a_linears[n].bias.detach(), math_mode),
         }
+        H = self.n_heads
+        if math_mode == L.MATH_F16F8 and d == 128 * H and H % 2 == 0 and H <= 8:
+            P["ntgt_qkv_heads"] = P["ntgt_qkv"].permuted(head_interleave(H, 128).to(P["ntgt_qkv"].W.device))
         if rot is not None and self.use_deferred_ln and math_mode == L.MATH_F16F8 and rot.shape[0] == rot.shape[1]:
             r64 = rot.detach().double()
             eye = torch.eye(r64.shape[0], dtype=r64.dtype, device=r64.device)
@@ -314,21 +339,31 @@ class HGTLayer(hetero.IncrementalState, nn.Module):
             ops.edge_attn(q, k, v, G.nn_indptr, G.nn_indices, H, t_agg, n_dst_dev=n_dev, tag=tag)
         return as_act(t_agg, P["math"])
 
+    def _full_attn(self, P, G: TokenGraph, h_n, n_dev):
+        """Q|K'|V' of all ntgt nodes -> chain attention -> the A-linear operand.  One kernel (ops.linear_f16f8_nn_attn) where it
+        applies: MATH_F16F8, d_k = 128, clusters of 1, 3, 5 or 7 nodes and an fp32 Q|K'|V'."""
+        d = P["d"]
+        x = with_q8(h_n, P["math"], n_dev)
+        hq = self._hq(G, h_n, centre=False)
+        if ("ntgt_qkv_heads" in P and self.use_fused_nn and self.use_cluster_kernel and not G.dedup and G.w in (1, 3, 5, 7) and not hq
+                and isinstance(x, ops.Split) and x.q8 is not None and ops.f16f8_supported(x.d)
+                and gemm_act(P["math"], x.shape[0], d, lo=False) == ops.HI_Q8):
+            W = P["ntgt_qkv_heads"]
+            return ops.linear_f16f8_nn_attn(x, W.W, W.w8(), W.b, G, self.n_heads, w_scale=W.scale)
+        qkv = _lin(x, P["ntgt_qkv"], P["math"], m_dev=n_dev, out_dtype=_attn_in_dtype(P["math"], hq))
+        return self._nn_attn(P, G, qkv[:, :d], qkv[:, d:2 * d], qkv[:, 2 * d:], h_n.shape[0], centre=False, n_dev=n_dev, c_dev=None)
+
     def ntgt_full(self, P, G: TokenGraph, h_n, n_dev):
         """All ntgt nodes: Q|K'|V' -> chain attention -> A-linear + residual + LN."""
-        d = P["d"]
-        qkv = _lin(with_q8(h_n, P["math"], n_dev), P["ntgt_qkv"], P["math"], m_dev=n_dev, out_dtype=_attn_in_dtype(P["math"], self._hq(G, h_n, centre=False)))
-        t_agg = self._nn_attn(P, G, qkv[:, :d], qkv[:, d:2 * d], qkv[:, 2 * d:], h_n.shape[0], centre=False, n_dev=n_dev,
-                              c_dev=None)
+        t_agg = self._full_attn(P, G, h_n, n_dev)
         return self._out(P, P["n"], t_agg, h_n, n_dev, feeds_gemm=True)        # h of the next layer: a GEMM operand
 
     def ntgt_full_deferred(self, P, G: TokenGraph, x_n, n_dev):
         """ntgt_full of layer 0 with the rotation folded and the LayerNorm DEFERRED: returns (z', stats) -- the pre-norm sum in the
         un-rotated basis as a GEMM operand and (mean, 1 / std) of its rotation per node (ops.rowstats_q8) -- instead of h1.  The
         residual x is added un-rotated (z' = A-linear(t) rot + x), which halves the output projection (K = d instead of 2 d)."""
-        d, D = P["d"], P["defer"]
-        qkv = _lin(with_q8(x_n, P["math"], n_dev), P["ntgt_qkv"], P["math"], m_dev=n_dev, out_dtype=_attn_in_dtype(P["math"], self._hq(G, x_n, centre=False)))
-        t_agg = self._nn_attn(P, G, qkv[:, :d], qkv[:, d:2 * d], qkv[:, 2 * d:], x_n.shape[0], centre=False, n_dev=n_dev, c_dev=None)
+        D = P["defer"]
+        t_agg = self._full_attn(P, G, x_n, n_dev)
         o = _lin(with_q8(t_agg, P["math"], n_dev), D["a"], P["math"], m_dev=n_dev)
         return ops.rowstats_q8(o, x_n, D["u"], P["ln"][P["n"]][2], n_dev)
 

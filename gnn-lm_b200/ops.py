@@ -184,6 +184,42 @@ def linear_f16f8(A1: Split, W_hi, W8, bias=None, *, A2: Optional[Split] = None, 
     return out
 
 
+def nn_window_plan(M: int, w: int):
+    """Row windows of linear_f16f8_nn_attn for M rows and clusters of at most w nodes: window j loads the 128 rows starting at
+    j S - h and owns [j S, j S + S), h = w - 1, S = 128 - 2h.  Returns (h, S, number of windows)."""
+    h = w - 1
+    S = 128 - 2 * h
+    return h, S, -(-M // S)
+
+
+_NN_ERR = {}
+
+
+def nn_attn_error(device) -> torch.Tensor:
+    """The error word of linear_f16f8_nn_attn on `device` (int32 [1]): set to 1, and never cleared by the kernel, when a node's
+    chain edges do not fit its window -- more than three edges, or a neighbour more than w - 1 ids away."""
+    dev = torch.device(device)
+    if dev not in _NN_ERR:
+        _NN_ERR[dev] = torch.zeros(1, dtype=torch.int32, device=dev)
+    return _NN_ERR[dev]
+
+
+def linear_f16f8_nn_attn(A: Split, W_hi, W8, bias, G, H: int, *, w_scale=1.0):
+    """Chain attention of every ntgt node of G (gnnlm_hgt_cluster_attn's all-nodes form) fused into the epilogue of its
+    Q | K' | V' projection: W_hi / W8 / bias hold the projection's rows in head-interleaved order (hgt.head_interleave).  Returns
+    the attention output [M, d] as the operand of the next linear_f16f8 (fp16 hi + e4m3 companion); Q | K' | V' are never written.
+    The live row count is G's."""
+    M, K = A.shape
+    N = W_hi.shape[0]
+    assert A.q8 is not None and N % 3 == 0 and W_hi.shape[1] == K and W8.shape == (N, 2 * K) and W_hi.dtype == torch.float16
+    out = empty_act(M, N // 3, HI_Q8, W_hi.device)
+    L.call("gnnlm_linear_f16f8_nn_attn", L.ptr(A.data), L.ptr(A.q8), A.data.stride(0), A.q8.stride(0), K, L.ptr(W_hi), L.ptr(W8),
+           float(w_scale), W_hi.stride(0), W8.stride(0), L.ptr(bias), L.ptr(G.nn_indptr), L.ptr(G.nn_indices), G.w, H,
+           L.ptr(out.data), out.data.stride(0), L.ptr(out.q8), out.q8.stride(0), L.ptr(nn_attn_error(W_hi.device)), M,
+           L.ptr(G.n_ntgt_dev), L.stream_ptr(), tag=f"nn_full[{N}x{K}]", work=(M, N, K))
+    return out
+
+
 def linear_lse(A, W, pick, *, W_lo=None, m_dev=None, math=L.MATH_FP32_SIMT, w_scale=1.0):
     """Row log-sum-exp partials + picked column of A @ W^T without materialising it."""
     a_ptr, a_code, lda, K = _mat(A)

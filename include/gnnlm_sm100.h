@@ -239,6 +239,18 @@ int32_t gnnlm_linear_f16f8(const void* A1, const void* A1q, int64_t lda1, int64_
                            const void* A2q, int64_t lda2, int64_t ldq2, int64_t K2, const void* W_hi, const void* W8,
                            float w_scale, int64_t ldw, int64_t ldw8, const float* bias, void* C, int32_t c_dtype, int64_t ldc,
                            int64_t M, const int32_t* m_dev, int64_t N, void* C8, gnnlm_stream_t stream);
+/* The all-nodes ntgt-intra-ntgt chain attention of gnnlm_hgt_cluster_attn_q8 (write_lo = 0) fused into the epilogue of its
+ * Q | K' | V' projection: Q | K' | V' are never written.  A / Aq: split-fp16 operand [M, K] (hi half read) and its e4m3 companion;
+ * W_hi / W8 / bias: the projection with its rows in head-interleaved order [Q_0 | K'_0 | ... | Q_{H-1} | K'_{H-1} | V'_0 .. V'_{H-1}],
+ * d_k = 128, N = 3 H d_k, H even and <= 8.  nn_indptr / nn_indices: the chain edges of every ntgt node ([left,] self[, right]) of a
+ * graph whose clusters have at most max_cluster (1, 3, 5 or 7) nodes.  out [M, ldo] fp16: hi half of the result; q8 [M, ldq8]:
+ * its e4m3 companion (the operand set gnnlm_linear_f16f8 reads).  *err is set to 1 (never cleared) when a node has more than three
+ * chain edges or a neighbour more than max_cluster - 1 ids away. */
+int32_t gnnlm_linear_f16f8_nn_attn(const void* A, const void* Aq, int64_t lda, int64_t ldq, int64_t K, const void* W_hi,
+                                   const void* W8, float w_scale, int64_t ldw, int64_t ldw8, const float* bias,
+                                   const int32_t* nn_indptr, const int32_t* nn_indices, int32_t max_cluster, int32_t H, void* out,
+                                   int64_t ldo, void* q8, int64_t ldq8, int32_t* err, int64_t M, const int32_t* m_dev,
+                                   gnnlm_stream_t stream);
 
 /* Same contraction, but instead of storing C the epilogue keeps, per row and per column tile,
  * (max, sum exp(x - max)) and the single column `pick[m]` -- the [rows, vocab] tensor of
